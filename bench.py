@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 10 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference            # the reference's own CPU path on the host cores
+    python bench.py --dump-outputs DIR          # also write a sample of the timed step's outputs to DIR/*.npy
 
 Workload (BASELINE.json configs[1]): batched forward + inverse negacyclic NTT,
 N = 2^16, 55-bit prime (GeneratePrimes(1, 55, true, N)), 8192 polynomials per GPU,
@@ -64,7 +65,13 @@ def parse():
     ap.add_argument("--no-eltwise", action="store_true")
     ap.add_argument("--no-composites", action="store_true", help="skip the c4 / c5 legs")
     ap.add_argument("--e2e-steps", type=int, default=None)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of what the last one computed to DIR/*.npy "
+                         "(b200 arm, rank 0)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 # ------------------------------------------------------------------ clocks
@@ -283,6 +290,21 @@ def gpu_time_ms(torch, fn, reps, sync):
     return e0.elapsed_time(e1) / reps
 
 
+def dump_outputs(out_dir, np, torch, outputs, budget=16 << 20):
+    """Write each (batch, N) result of the timed step as <out_dir>/<name>.npy, so that two builds run with the same
+    arguments (hence the same seeded inputs) can be compared output for output.  A fixed sample of rows is kept
+    (numpy default_rng(0), at most `budget` bytes per output), in float64 of shape (rows, N, 2): the high and the low
+    32 bits of every 64-bit word, because float64 alone would round residues above 2^53."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        batch, n = t.shape
+        rows = min(batch, max(1, budget // (16 * n)))
+        idx = np.sort(np.random.default_rng(0).choice(batch, size=rows, replace=False))
+        w = t[torch.from_numpy(idx).to(t.device)].cpu().numpy().view(np.uint64)
+        halves = np.stack([w >> np.uint64(32), w & np.uint64(0xFFFFFFFF)], axis=-1).astype(np.float64)
+        np.save(os.path.join(out_dir, f"{name}.npy"), halves)
+
+
 def eltwise_sweep(hb, torch, peak, gen, sync):
     """BASELINE configs[2]: N = 2^10..2^17 x q in {40,50,60}-bit x {MultMod, FMAMod, ReduceMod}, batch 4096"""
     out = {"batch": 4096, "bytes_per_element": {"mult_mod": 24, "fma_mod": 24, "reduce_mod": 16}, "points": []}
@@ -374,11 +396,13 @@ def c4_leg(args, hb, torch, rank, world, gen, sync, peak, cpu_ok):
         polys = max(threads, 8)
         x = np.random.default_rng(1).integers(0, q, size=n * polys, dtype=np.uint64)
         y = np.random.default_rng(2).integers(0, q, size=n * polys, dtype=np.uint64)
+        # only the compiled reference splits an element-wise call over threads; the C restatement runs it on one
+        split = {"rows": polys, "threads": threads} if chk.kind == "reference" else {}
 
         def cpu():
             fx = chk.ntt_forward(x, n, q, 1, 4, threads=threads)
             fy = chk.ntt_forward(y, n, q, 1, 4, threads=threads)
-            p = chk.mult_mod(fx, fy, q, 4, rows=polys, threads=threads)
+            p = chk.mult_mod(fx, fy, q, 4, **split)
             return chk.ntt_inverse(p, n, q, 1, 1, threads=threads)
         cpu()
         t0 = time.perf_counter()
@@ -556,6 +580,8 @@ def run_b200_arm(args):
     ms_total = e0.elapsed_time(e1)
     launches = hb.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, np, torch, {"ntt_forward": y, "ntt_inverse": z})
     ms_total = max_over_ranks(ms_total, world)
     ms_step = ms_total / args.steps
     value = whole_job_value(2 * batch, world, ms_step * 1e-3)

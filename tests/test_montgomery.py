@@ -5,7 +5,7 @@ on the GPU -- the element-wise kernels against the checker."""
 import numpy as np
 import pytest
 
-from util import uniform_below
+from util import sha, uniform_below
 
 MASK64 = (1 << 64) - 1
 # (modulus, r, T, T * 2^-r mod modulus): restated from the reference's tests
@@ -21,6 +21,20 @@ def _cases():
             (769, 10), (5, 3)]
 
 
+def _kat_arrays(q, r):
+    """operands a, b (0, 1 and q-1 first), R^2 mod q, and the known answers a*b/R, a*R and a*b mod q"""
+    R = 1 << r
+    n = 1031
+    a, b = uniform_below(q % 1000, n, q), uniform_below(q % 1000 + 1, n, q)
+    a[:3] = [0, 1, q - 1]
+    b[:3] = [q - 1, q - 1, q - 1]
+    rinv = pow(R, -1, q)
+    exp_mul = np.array([int(x) * int(y) * rinv % q for x, y in zip(a, b)], dtype=np.uint64)
+    exp_fin = np.array([int(x) * R % q for x in a], dtype=np.uint64)
+    plain = np.array([int(x) * int(y) % q for x, y in zip(a, b)], dtype=np.uint64)
+    return a, b, R * R % q, exp_mul, exp_fin, plain
+
+
 def _check_impl(impl):
     assert impl.hensel_lemma_2adic_root(46, 67280421310725) == 62463730494515  # test-avx512-util.cpp:417
     for q, r, T, out in REDC_KATS:
@@ -29,19 +43,11 @@ def _check_impl(impl):
         assert impl.montgomery_reduce(T >> 64, T & MASK64, q, r, inv) == out, (q, r, T)
     for q, r in _cases():
         inv = impl.hensel_lemma_2adic_root(r, q)
-        R = 1 << r
-        r2 = R * R % q
-        n = 1031
-        a, b = uniform_below(q % 1000, n, q), uniform_below(q % 1000 + 1, n, q)
-        a[:3] = [0, 1, q - 1]
-        b[:3] = [q - 1, q - 1, q - 1]
-        rinv = pow(R, -1, q)
-        exp_mul = np.array([int(x) * int(y) * rinv % q for x, y in zip(a, b)], dtype=np.uint64)
+        a, b, r2, exp_mul, exp_fin, plain = _kat_arrays(q, r)
         assert (impl.mont_reduce_mod(a, b, q, r, inv) == exp_mul).all(), (q, r)
         fin = impl.montgomery_form_in(a, r2, q, r, inv)
-        assert (fin == np.array([int(x) * R % q for x in a], dtype=np.uint64)).all(), (q, r)
+        assert (fin == exp_fin).all(), (q, r)
         assert (impl.montgomery_form_out(fin, q, r, inv) == a).all(), (q, r)               # test-eltwise-reduce-mod-avx512.cpp:59-64
-        plain = np.array([int(x) * int(y) % q for x, y in zip(a, b)], dtype=np.uint64)
         assert (impl.mont_reduce_mod(fin, b, q, r, inv) == plain).all(), (q, r)            # test-eltwise-mult-mod-avx512.cpp:229-236
 
 
@@ -49,17 +55,25 @@ def test_restatement_against_the_reference_kats(port):
     _check_impl(port)
 
 
-def test_compiled_reference_against_its_own_kats_and_the_restatement(ref, port):
-    if not getattr(ref, "has_mont", False):
-        pytest.skip("oracle/_ref was built before the Montgomery veneer existed")
-    _check_impl(ref)
+def test_compiled_reference_against_its_own_kats_and_the_restatement(reference_outputs, port):
+    """What the compiled reference returned (tests/golden/reference_outputs.json: scalars, and SHA-256 of arrays)
+    against the known answers, and against the restatement on random inputs."""
+    ref = reference_outputs["montgomery"]
+    assert ref["hensel_lemma_2adic_root(46, 67280421310725)"] == 62463730494515   # test-avx512-util.cpp:417
+    assert ref["montgomery_reduce"] == [out for *_, out in REDC_KATS]
     for q, r in _cases():
-        inv = ref.hensel_lemma_2adic_root(r, q)
-        assert inv == port.hensel_lemma_2adic_root(r, q)
+        c = ref["cases"][f"{q},{r}"]
+        inv = port.hensel_lemma_2adic_root(r, q)
+        assert c["inv"] == inv
+        a, b, _, exp_mul, exp_fin, plain = _kat_arrays(q, r)
+        assert c["kat mont_reduce_mod"] == sha(exp_mul), (q, r)
+        assert c["kat montgomery_form_in"] == sha(exp_fin), (q, r)
+        assert c["kat montgomery_form_out"] == sha(a), (q, r)
+        assert c["kat mont_reduce_mod of form_in"] == sha(plain), (q, r)
         a, b = uniform_below(3, 4099, q), uniform_below(4, 4099, q)
-        assert (ref.mont_reduce_mod(a, b, q, r, inv) == port.mont_reduce_mod(a, b, q, r, inv)).all()
-        if r in (46, 61) and ref.avx512:
-            assert ref.last_mont_was_avx512  # the reference's own AVX-512 helper produced these bits
+        assert c["mont_reduce_mod"] == sha(port.mont_reduce_mod(a, b, q, r, inv)), (q, r)
+        if r in (46, 61) and ref["avx512"]:
+            assert c["avx512 helper"]  # the reference's own AVX-512 helper produced these bits
 
 
 def test_product_host_functions(hb):
@@ -121,15 +135,26 @@ def test_montgomery_kernels_match_the_checker(hb, checker):
     assert (host(out[1:]) == checker.montgomery_form_out(a[:1024], q, r, inv)).all()
 
 
+RADIX4_CASES = ((4, 30), (5, 40), (10, 50), (11, 55), (12, 60), (13, 61), (15, 45), (16, 55), (17, 60))
+
+
+def radix4_inputs(logn, q):
+    """("forward" | "inverse", in_mf, out_mf, x) of every transform compared with the reference's radix-4 path"""
+    n = 1 << logn
+    for in_mf, out_mf in ((1, 1), (4, 1), (2, 4)):
+        yield "forward", in_mf, out_mf, uniform_below(logn + in_mf, n, q * in_mf)
+    for in_mf, out_mf in ((1, 1), (2, 1), (2, 2)):
+        yield "inverse", in_mf, out_mf, uniform_below(logn + 7 + in_mf, n, q * in_mf)
+
+
 @pytest.mark.gpu
-def test_ntt_matches_the_references_radix4_path(hb, checker):
+def test_ntt_matches_the_references_radix4_path(hb, reference_outputs):
     """The register passes of the sm_100a kernels consume twiddles by the reference's radix-4 index rule
     (W[m+i], W[2(m+i)], W[2(m+i)+1] = a tree node and its two children, ntt-radix-4.cpp:223-233; odd log2 N starts
     with one radix-2 stage, :49-71): their outputs must equal ForwardTransformToBitReverseRadix4 /
-    InverseTransformFromBitReverseRadix4 of the compiled reference bit for bit (lazy outputs mod q)."""
+    InverseTransformFromBitReverseRadix4 of the compiled reference bit for bit (lazy outputs mod q).  The reference's
+    outputs are recorded in tests/golden/reference_outputs.json (SHA-256; of the residues mod q for lazy outputs)."""
     torch = pytest.importorskip("torch")
-    if not hasattr(checker, "ntt_forward_radix4"):
-        pytest.skip("the radix-4 entry points need the compiled reference")
 
     def dev(a):
         return torch.from_numpy(np.ascontiguousarray(a, dtype=np.uint64).view(np.int64)).cuda()
@@ -137,23 +162,17 @@ def test_ntt_matches_the_references_radix4_path(hb, checker):
     def host(t):
         return t.cpu().numpy().view(np.uint64)
 
-    for logn, bits in ((4, 30), (5, 40), (10, 50), (11, 55), (12, 60), (13, 61), (15, 45), (16, 55), (17, 60)):
+    for logn, bits in RADIX4_CASES:
+        ref = reference_outputs["radix4"][f"{logn},{bits}"]
         n = 1 << logn
         q = hb.GeneratePrimes(1, bits, True, n)[0]
+        assert q == ref["q"]
         t = hb.NTT(n, q)
-        for in_mf, out_mf in ((1, 1), (4, 1), (2, 4)):
-            x = uniform_below(logn + in_mf, n, q * in_mf)
-            exp = checker.ntt_forward_radix4(x, n, q, in_mf, out_mf)
-            got = host(t.ComputeForward(dev(np.zeros_like(x)), dev(x), in_mf, out_mf))
+        for direction, in_mf, out_mf, x in radix4_inputs(logn, q):
+            fn = t.ComputeForward if direction == "forward" else t.ComputeInverse
+            got = host(fn(dev(np.zeros_like(x)), dev(x), in_mf, out_mf))
+            exp = ref[direction][f"{in_mf},{out_mf}"]
             if out_mf == 1:
-                assert (got == exp).all(), ("fwd", logn, in_mf)
+                assert sha(got) == exp, (direction, logn, in_mf)
             else:
-                assert (got % np.uint64(q) == exp % np.uint64(q)).all() and (got < np.uint64(4 * q)).all()
-        for in_mf, out_mf in ((1, 1), (2, 1), (2, 2)):
-            x = uniform_below(logn + 7 + in_mf, n, q * in_mf)
-            exp = checker.ntt_inverse_radix4(x, n, q, in_mf, out_mf)
-            got = host(t.ComputeInverse(dev(np.zeros_like(x)), dev(x), in_mf, out_mf))
-            if out_mf == 1:
-                assert (got == exp).all(), ("inv", logn, in_mf)
-            else:
-                assert (got % np.uint64(q) == exp % np.uint64(q)).all() and (got < np.uint64(2 * q)).all()
+                assert sha(got % np.uint64(q)) == exp and (got < np.uint64(out_mf * q)).all(), (direction, logn, in_mf)
